@@ -90,7 +90,12 @@ def parse():
                                                         "(on by default for N > 1; untimed, ~2 s)")
   ap.add_argument("--no-verify", action="store_true")
   ap.add_argument("--layer-table", action="store_true", help="add the live per-geometry conv table to roofline.by_layer")
+  ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                  help="write what the last timed step returned and left in the network (losses, parameters, buffers, "
+                       "gradients) as DIR/<name>.npy, to compare two builds output for output")
   a = ap.parse_args()
+  if a.dump_outputs and a.impl != "ours":
+    ap.error("--dump-outputs records this repo's timed path (--impl ours)")
   if a.head is None:
     a.head = "A" if CONFIGS[a.config]["kind"] == "seg" else "B"
   return a
@@ -301,10 +306,9 @@ def run_reference(args):
   if rank != 0:
     return
   pairs = args.cpu_pairs or CONFIGS[args.config]["cpu_pairs"]
-  steps = max(1, min(args.steps, 4))  # bounded sample: a step is seconds of CPU work
-  base, dt = time_cpu_reference(args, pairs, steps, 1)
+  base, dt = time_cpu_reference(args, pairs, args.steps, args.warmup)
   line = {"impl": "reference", "metric": METRIC, "value": base["value"], "unit": "img-pairs/s", "n_gpus": args.gpus,
-          "steps": steps, "warmup": 1, "ms_per_step": dt * 1e3, "higher_is_better": True,
+          "steps": args.steps, "warmup": max(1, args.warmup), "ms_per_step": dt * 1e3, "higher_is_better": True,
           "scaling": CONFIGS[args.config]["scaling"], "vs_baseline": None, "dtype": "f32", "data": "synthetic",
           "config": workload_config(args, pairs, 1), "cpu_baseline": base,
           "e2e": {"value": base["value"], "unit": "img-pairs/s", "h2d_bytes_per_step": 0, "d2h_bytes_per_step": 0},
@@ -352,8 +356,45 @@ class Job(object):
                             arena=self.arena)
 
 
-def measure(job, resident, host, steps, warmup, world, dev, sampler=None):
-  """-> dict(sec, sec_e2e, launches, loss, clocks): device-timed (CUDA events, max over ranks) resident and e2e legs."""
+DUMP_SAMPLE = 1 << 15  # entries kept of a larger tensor by --dump-outputs
+DUMP_LIMIT = 64 << 20  # bytes --dump-outputs may write
+
+
+def dump_outputs(job, out, path):
+  """Writes what a step handed its caller: the returned (loss, loss_no_lamb), and the parameters, buffers and gradients
+  it left in the network, as float32 (integer buffers: float64) .npy files.  A tensor of more than DUMP_SAMPLE entries
+  is reduced to DUMP_SAMPLE of its flat entries, at sorted indices drawn by a generator seeded with the tensor's name,
+  so the sample is the same in every run and every build."""
+  import zlib
+
+  import numpy as np
+  import torch
+  arrays = {"loss": out[0], "loss_no_lamb": out[1]}
+  for n, p in job.net.named_parameters():
+    arrays["param." + n] = p
+    if p.grad is not None:
+      arrays["grad." + n] = p.grad
+  for n, b in job.net.named_buffers():
+    arrays["buffer." + n] = b
+  os.makedirs(path, exist_ok=True)
+  total = 0
+  for name, t in arrays.items():
+    a = t.detach().reshape(-1)
+    if a.numel() > DUMP_SAMPLE:
+      rng = np.random.default_rng(zlib.crc32(name.encode()))
+      idx = np.sort(rng.choice(a.numel(), DUMP_SAMPLE, replace=False))
+      a = a[torch.from_numpy(idx).to(a.device)]
+    a = (a.float() if t.is_floating_point() else a.double()).cpu().numpy()
+    if t.numel() <= DUMP_SAMPLE:
+      a = a.reshape(tuple(t.shape))
+    total += a.nbytes
+    assert total <= DUMP_LIMIT, "--dump-outputs: more than %d bytes" % DUMP_LIMIT
+    np.save(os.path.join(path, name + ".npy"), a)
+
+
+def measure(job, resident, host, steps, warmup, world, dev, sampler=None, dump=None):
+  """-> dict(sec, sec_e2e, launches, loss, clocks): device-timed (CUDA events, max over ranks) resident and e2e legs.
+  ``dump``: directory for dump_outputs of the last resident step (rank 0)."""
   import torch
   import torch.distributed as dist
 
@@ -392,6 +433,8 @@ def measure(job, resident, host, steps, warmup, world, dev, sampler=None):
   if getattr(job, "gstep", None) is not None:  # replays do not pass through the host-side counter
     launches += steps * job.gstep.launches_per_replay
   clocks = sampler.stop() if sampler is not None else None
+  if dump is not None:
+    dump_outputs(job, last, dump)
   job.step(host)
   sec_e, _, _ = timed(host, True)
   return dict(sec=sec, sec_e2e=sec_e, launches=launches, loss=float(last[0]), clocks=clocks, wall=wall)
@@ -553,7 +596,8 @@ def run_ours(args):
   host = make_host_batch(args, B, 1000 + rank)
   resident = [h.to(dev) for h in host]
   job = Job(args, args.precision, dev)
-  m = measure(job, resident, host, args.steps, args.warmup, world, dev, ClockSampler(local) if rank == 0 else None)
+  m = measure(job, resident, host, args.steps, args.warmup, world, dev, ClockSampler(local) if rank == 0 else None,
+              args.dump_outputs if rank == 0 else None)
   value = B * world * args.steps / m["sec"]
   e2e = B * world * args.steps / m["sec_e2e"]
 

@@ -1,6 +1,8 @@
 """Builds iic_b200/lib/libiic_b200.so (the C-ABI library) with nvcc for sm_100a.
 
-nvcc cross-compiles without a GPU.  Objects are cached under build/ keyed by source mtime.
+nvcc cross-compiles without a GPU.  Objects are cached under build/ keyed by source mtime.  Every output is written
+under a temporary name and renamed into place, so processes building at the same time (e.g. test workers) never
+read a half-written object or library.
 """
 import os
 import subprocess
@@ -33,9 +35,11 @@ def _compile(src):
   deps = [s, os.path.join(ROOT, "include", "iic_b200.h")] + [os.path.join(CSRC, h) for h in os.listdir(CSRC) if h.endswith(".cuh")]
   if not any(_newer(d, o) for d in deps):
     return o, ""
-  r = subprocess.run([NVCC] + FLAGS + ["-c", s, "-o", o], capture_output=True, text=True)
+  tmp = "%s.%d.tmp" % (o, os.getpid())
+  r = subprocess.run([NVCC] + FLAGS + ["-c", s, "-o", tmp], capture_output=True, text=True)
   if r.returncode != 0:
     raise RuntimeError("nvcc failed for %s:\n%s\n%s" % (src, r.stdout, r.stderr))
+  os.replace(tmp, o)
   return o, r.stderr
 
 
@@ -50,9 +54,11 @@ def build(verbose=False):
       if log:
         print(log)
   if any(_newer(o, LIB) for o in objs):
-    r = subprocess.run([NVCC, "-shared", "-o", LIB] + objs + ["-lcudart"], capture_output=True, text=True)
+    tmp = "%s-%d.so" % (LIB[:-3], os.getpid())
+    r = subprocess.run([NVCC, "-shared", "-o", tmp] + objs + ["-lcudart"], capture_output=True, text=True)
     if r.returncode != 0:
       raise RuntimeError("link failed:\n%s\n%s" % (r.stdout, r.stderr))
+    os.replace(tmp, LIB)
   return LIB
 
 

@@ -1,7 +1,8 @@
-"""Import shim that loads the UNMODIFIED reference modules from /root/reference
-(Python-2.7 / torch-0.4.1 code) under Python 3 / torch 2.x.  Only usable in the
-build container; used by tests/golden/make_golden.py and by the (skipped when
-absent) oracle-vs-reference tests.  Recipe: SURVEY.md Appendix A.
+"""Import shim that loads the UNMODIFIED reference modules (xu-ji/IIC, Python-2.7 /
+torch-0.4.1 code; a checkout named by $IIC_REFERENCE) under Python 3 / torch 2.x.
+Used only by tests/golden/make_golden.py, which records what the reference
+computes as the golden fixtures the tests compare against.  Recipe: SURVEY.md
+Appendix A.
 """
 import builtins
 import importlib

@@ -267,12 +267,74 @@ def gen_precision(ref, out):
     print("precision fixture", sz, pairs, head, loss.item())
 
 
+def live_iid_inputs():
+  z, zt = softmax_pair("live", 333, 13, corr=0.4)
+  return z, zt, 1.2
+
+
+def sparse_inputs():
+  """Input of random_translation_multiple, and inputs of the segmentation losses with a sparse displacement window."""
+  return weights.normal("sparse.x", (2, 3, 12, 12)), seg_inputs("seg.sparse", 3, 4, 16, flips=True)
+
+
+SPARSE_SEEDS = range(6)  # np.random.seed before each random_translation_multiple(x, 2, 4)
+SPARSE_LOSS_SEED = 11  # np.random.seed before each loss call
+SPARSE_LOSS_KW = dict(lamb=1.2, half_T_side_dense=2, half_T_side_sparse_min=1, half_T_side_sparse_max=3)
+
+# networks whose reference state_dict layout (key order, shapes, dtypes) a checkpoint carries
+CHECKPOINT_SPECS = {
+  "ClusterNet5gTwoHead": dict(in_channels=2, input_sz=32, num_sub_heads=3, output_k_A=20, output_k_B=5, batchnorm_track=True),
+  "ClusterNet6cTwoHead": dict(in_channels=1, input_sz=24, num_sub_heads=2, output_k_A=12, output_k_B=4, batchnorm_track=False),
+  "SegmentationNet10aTwoHead": dict(in_channels=5, input_sz=32, num_sub_heads=1, output_k_A=6, output_k_B=3, batchnorm_track=True),
+}
+
+
+def gen_calls(ref, out):
+  """Single calls into the reference whose results the oracle must reproduce exactly: IID_loss, the seeded sparse
+  displacement of the segmentation losses, and the state_dict layout a reference checkpoint has."""
+  from oracle import seg_losses
+  z, zt, lamb = live_iid_inputs()
+  with torch.no_grad():
+    r = ref.IID_loss(z.clone(), zt.clone(), lamb=lamb)
+  out["iid_live/ref_loss"] = np.float32(r[0])
+  out["iid_live/ref_loss_no_lamb"] = np.float32(r[1])
+  o = iid_losses.IID_loss(z, zt, lamb=lamb)
+  assert float(r[0]) == float(o[0]) and float(r[1]) == float(o[1])
+  x, (x1, x2, theta, mask) = sparse_inputs()
+  shifted = []
+  for seed in SPARSE_SEEDS:
+    np.random.seed(seed)
+    shifted.append(ref.random_translation_multiple(x, 2, 4))
+    np.random.seed(seed)
+    assert torch.equal(shifted[-1], seg_losses.random_translation_multiple(x, 2, 4))
+  out["sparse/ref_translated"] = torch.stack(shifted).numpy()
+  for fn_name in ("IID_segmentation_loss", "IID_segmentation_loss_uncollapsed"):
+    np.random.seed(SPARSE_LOSS_SEED)
+    a, b = x1.clone().requires_grad_(True), x2.clone().requires_grad_(True)
+    l, l1 = getattr(ref, fn_name)(a, b, all_affine2_to_1=theta, all_mask_img1=mask, **SPARSE_LOSS_KW)
+    ga, gb = torch.autograd.grad(l, [a, b])
+    p = "sparse/%s/" % fn_name
+    out[p + "ref_loss"] = np.float32(l.item())
+    out[p + "ref_loss_no_lamb"] = np.float32(l1.item())
+    out[p + "ref_dx1"] = ga.numpy()
+    out[p + "ref_dx2"] = gb.numpy()
+    print("sparse", fn_name, l.item(), l1.item())
+  for name, cfg in CHECKPOINT_SPECS.items():
+    sd = getattr(ref, name)(Namespace(**cfg)).state_dict()
+    p = "checkpoint/%s/" % name
+    out[p + "keys"] = np.array(list(sd))
+    out[p + "shapes"] = np.array([",".join(map(str, v.shape)) for v in sd.values()])
+    out[p + "dtypes"] = np.array([str(v.dtype).replace("torch.", "") for v in sd.values()])
+    print("checkpoint", name, len(sd), "entries")
+
+
 def main():
   assert refshim.available(), "needs /root/reference"
   ref = refshim.load()
   only = sys.argv[1:]
   for fname, gens in [("iid_loss.npz", [gen_iid]), ("seg_loss.npz", [gen_seg]),
-                      ("nets.npz", [gen_nets, gen_seg_nets]), ("precision.npz", [gen_precision])]:
+                      ("nets.npz", [gen_nets, gen_seg_nets]), ("precision.npz", [gen_precision]),
+                      ("reference_calls.npz", [gen_calls])]:
     if only and fname not in only:
       continue
     out = {}

@@ -34,7 +34,9 @@ def test_library_exports_every_declared_symbol(built):
 
 
 def test_sm100a_tensor_core_and_async_copy_sass(built):
-  sass = subprocess.run(["cuobjdump", "-sass", built], capture_output=True, text=True, check=True).stdout
+  from iic_b200 import build
+  cuobjdump = os.path.join(os.path.dirname(build.NVCC), "cuobjdump")  # the toolkit that built the library
+  sass = subprocess.run([cuobjdump, "-sass", built], capture_output=True, text=True, check=True).stdout
   assert "UTCHMMA" in sass, "tcgen05.mma missing from the SASS"
   assert "LDTM" in sass and "UTMALDG" in sass and "UTMASTG" in sass  # TMEM read-out, TMA loads (tiled + im2col) and stores
   assert "UTMALDG.4D.IM2COL" in sass
@@ -81,7 +83,7 @@ def test_missing_library_fails_loudly(monkeypatch):
     _lib.lib()
 
 
-def test_default_kernel_variants_are_the_validated_set():
+def test_default_kernel_variants_are_the_validated_set(built):
   """The defaults that ship are the set measured fastest on a B200 with the whole GPU suite green
   (profiles/r01_bench_v10_variants.md); variants written after the last GPU session must stay off until they have run
   on hardware (DESIGN.md S8)."""

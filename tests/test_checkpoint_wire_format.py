@@ -1,38 +1,44 @@
 """SURVEY.md S8f row 3: a checkpoint written by the reference's own modules (state_dict of the unmodified reference net,
 optimiser state of torch.optim.Adam) loads into the iic_b200 network / FusedAdam with the reference's own calls, and
-back.  CPU only (modules hold parameters; no kernel runs)."""
+back.  The reference nets' state_dict layouts (key order, shapes, dtypes) are recorded in tests/golden/
+reference_calls.npz.  CPU only (modules hold parameters; no kernel runs)."""
 import collections
 import os
+import sys
 from argparse import Namespace
 
 import pytest
 import torch
 
-from oracle import refshim
-
-CFGS = {
-  "ClusterNet5gTwoHead": dict(in_channels=2, input_sz=32, num_sub_heads=3, output_k_A=20, output_k_B=5, batchnorm_track=True),
-  "ClusterNet6cTwoHead": dict(in_channels=1, input_sz=24, num_sub_heads=2, output_k_A=12, output_k_B=4, batchnorm_track=False),
-  "SegmentationNet10aTwoHead": dict(in_channels=5, input_sz=32, num_sub_heads=1, output_k_A=6, output_k_B=3, batchnorm_track=True),
-}
+sys.path.insert(0, os.path.join(os.path.dirname(__file__), "golden"))
+import make_golden  # noqa: E402
+from tests.conftest import load_golden  # noqa: E402
 
 
-@pytest.mark.skipif(not refshim.available(), reason="reference tree only exists in the build container")
-@pytest.mark.parametrize("name", sorted(CFGS))
+def _reference_checkpoint(name):
+  """A state_dict with the layout the reference net saves, filled with seeded values a fresh net does not hold."""
+  g = load_golden("reference_calls.npz").sub("checkpoint/" + name)
+  gen = torch.Generator().manual_seed(3)
+  sd = collections.OrderedDict()
+  for key, shape, dtype in zip(g["keys"], g["shapes"], g["dtypes"]):
+    shape, dtype = tuple(int(s) for s in str(shape).split(",") if s), getattr(torch, str(dtype))
+    if dtype.is_floating_point:
+      sd[str(key)] = torch.randn(shape, generator=gen).to(dtype)
+    else:
+      sd[str(key)] = torch.randint(1, 1000, shape, generator=gen).to(dtype)
+  return sd
+
+
+@pytest.mark.parametrize("name", sorted(make_golden.CHECKPOINT_SPECS))
 def test_reference_checkpoint_round_trip(name, tmp_path):
   import iic_b200.archs as archs
   from iic_b200.utils.checkpoint import load_into, load_reference_state_dict
-  ref = refshim.load()
-  torch.manual_seed(3)
-  rnet = getattr(ref, name)(Namespace(**CFGS[name]))
-  for b in rnet.buffers():  # make the BatchNorm buffers distinguishable from a fresh net's
-    if b.dtype.is_floating_point:
-      b.add_(torch.rand_like(b))
+  cfg = make_golden.CHECKPOINT_SPECS[name]
+  want = _reference_checkpoint(name)
   path = os.path.join(str(tmp_path), "latest_net.pytorch")
-  torch.save(rnet.state_dict(), path)  # cluster_sobel_twohead.py:429
-  net = archs.__dict__[name](Namespace(**CFGS[name]))
+  torch.save(want, path)  # cluster_sobel_twohead.py:429
+  net = archs.__dict__[name](Namespace(**cfg))
   net.load_state_dict(torch.load(path, map_location=lambda storage, loc: storage))  # :176-178, verbatim
-  want = rnet.state_dict()
   got = net.state_dict()
   assert list(got.keys()) == list(want.keys())
   for k in want:
@@ -40,15 +46,16 @@ def test_reference_checkpoint_round_trip(name, tmp_path):
   # saved from a DataParallel wrapper: keys carry a "module." prefix
   path2 = os.path.join(str(tmp_path), "dp.pytorch")
   torch.save(collections.OrderedDict(("module." + k, v) for k, v in want.items()), path2)
-  net2 = archs.__dict__[name](Namespace(**CFGS[name]))
+  net2 = archs.__dict__[name](Namespace(**cfg))
   load_into(net2, path2)
   assert all(torch.equal(net2.state_dict()[k], want[k]) for k in want)
   assert list(load_reference_state_dict(path2).keys()) == list(want.keys())
-  # and back: the reference module accepts what iic_b200 saves
+  # and back: what iic_b200 saves has the reference's layout (what its strict load_state_dict checks) and values
   torch.save(net.state_dict(), path)
-  rnet2 = getattr(ref, name)(Namespace(**CFGS[name]))
-  rnet2.load_state_dict(torch.load(path, map_location=lambda storage, loc: storage))
-  assert all(torch.equal(rnet2.state_dict()[k], want[k]) for k in want)
+  back = torch.load(path, map_location=lambda storage, loc: storage)
+  assert list(back.keys()) == list(want.keys())
+  for k in want:
+    assert back[k].shape == want[k].shape and back[k].dtype == want[k].dtype and torch.equal(back[k], want[k]), k
 
 
 def test_adam_state_interchanges_with_torch():

@@ -12,7 +12,8 @@ import torch
 
 sys.path.insert(0, os.path.join(os.path.dirname(__file__), "golden"))
 import make_golden  # noqa: E402  (specs + named input builders; imports no reference code)
-from oracle import iid_losses, nets, refshim, seg_losses, transforms, weights  # noqa: E402
+from oracle import iid_losses, nets, seg_losses, transforms, weights  # noqa: E402
+from tests.conftest import load_golden  # noqa: E402
 
 
 def test_iid_oracle_matches_reference_goldens(golden_iid):
@@ -47,14 +48,12 @@ def test_iid_known_answers():
   assert abs(iid_losses.IID_loss(zi, zti)[0].item()) < 5e-3
 
 
-@pytest.mark.skipif(not refshim.available(), reason="reference tree only exists in the build container")
 def test_iid_oracle_vs_live_reference():
-  ref = refshim.load()
-  z, zt = make_golden.softmax_pair("live", 333, 13, corr=0.4)
-  with torch.no_grad():
-    r = ref.IID_loss(z.clone(), zt.clone(), lamb=1.2)
-  o = iid_losses.IID_loss(z, zt, lamb=1.2)
-  assert float(r[0]) == float(o[0]) and float(r[1]) == float(o[1])
+  """One IID_loss call of the unmodified reference (recorded in tests/golden/reference_calls.npz): bit-identical."""
+  g = load_golden("reference_calls.npz").sub("iid_live")
+  z, zt, lamb = make_golden.live_iid_inputs()
+  o = iid_losses.IID_loss(z, zt, lamb=lamb)
+  assert float(g["ref_loss"]) == float(o[0]) and float(g["ref_loss_no_lamb"]) == float(o[1])
 
 
 def test_seg_oracle_matches_reference_goldens(golden_seg):
@@ -161,31 +160,25 @@ def test_grey_from_rgb_is_pil_L():
   assert torch.allclose(grey_from_rgb(f), (0.299 * f[:, 0] + 0.587 * f[:, 1] + 0.114 * f[:, 2])[:, None])
 
 
-@pytest.mark.skipif(not refshim.available(), reason="needs /root/reference (build container only)")
 def test_sparse_displacement_oracle_matches_reference_under_seed():
   """random_translation_multiple (seg transforms.py:146-166) and the losses that call it (seg IID_losses.py:29-32,
   :101-104): the oracle draws from numpy's global generator with the reference's calls, so the same seed gives the
-  same displacement, loss and gradients."""
-  ref = refshim.load()
-  x = weights.normal("sparse.x", (2, 3, 12, 12))
-  for seed in range(6):
-    np.random.seed(seed)
-    a = ref.random_translation_multiple(x, 2, 4)
+  same displacement, loss and gradients as the reference did (tests/golden/reference_calls.npz)."""
+  g = load_golden("reference_calls.npz").sub("sparse")
+  x, (x1, x2, theta, mask) = make_golden.sparse_inputs()
+  for i, seed in enumerate(make_golden.SPARSE_SEEDS):
     np.random.seed(seed)
     b = seg_losses.random_translation_multiple(x, 2, 4)
-    assert torch.equal(a, b)
-  x1, x2, theta, mask = make_golden.seg_inputs("seg.sparse", 3, 4, 16, flips=True)
+    assert torch.equal(torch.from_numpy(g["ref_translated"][i]), b)
   for fn_name in ("IID_segmentation_loss", "IID_segmentation_loss_uncollapsed"):
-    res = []
-    for mod in (ref, seg_losses):
-      np.random.seed(11)
-      a, b = x1.clone().requires_grad_(True), x2.clone().requires_grad_(True)
-      l, l1 = getattr(mod, fn_name)(a, b, all_affine2_to_1=theta, all_mask_img1=mask, lamb=1.2, half_T_side_dense=2,
-                                    half_T_side_sparse_min=1, half_T_side_sparse_max=3)
-      ga, gb = torch.autograd.grad(l, [a, b])
-      res.append((l.item(), l1.item(), ga, gb))
-    assert abs(res[0][0] - res[1][0]) < 1e-6 and abs(res[0][1] - res[1][1]) < 1e-6
-    assert torch.allclose(res[0][2], res[1][2], rtol=1e-4, atol=1e-8) and torch.allclose(res[0][3], res[1][3], rtol=1e-4, atol=1e-8)
+    want = g.sub(fn_name)
+    np.random.seed(make_golden.SPARSE_LOSS_SEED)
+    a, b = x1.clone().requires_grad_(True), x2.clone().requires_grad_(True)
+    l, l1 = getattr(seg_losses, fn_name)(a, b, all_affine2_to_1=theta, all_mask_img1=mask, **make_golden.SPARSE_LOSS_KW)
+    ga, gb = torch.autograd.grad(l, [a, b])
+    assert abs(float(want["ref_loss"]) - l.item()) < 1e-6 and abs(float(want["ref_loss_no_lamb"]) - l1.item()) < 1e-6
+    assert torch.allclose(torch.from_numpy(want["ref_dx1"]), ga, rtol=1e-4, atol=1e-8)
+    assert torch.allclose(torch.from_numpy(want["ref_dx2"]), gb, rtol=1e-4, atol=1e-8)
 
 
 def test_precision_fixture_oracle_matches_reference_golden():
