@@ -95,7 +95,11 @@ _SIGS = {
   "iic_avgpool_bwd": (c_int, [_P, _P, c_int, c_int, c_int, c_int, _P]),
   "iic_heads_fwd": (c_int, [_P, _P, _P, _P, _P, c_int, c_int, c_int, c_int, _P]),
   "iic_heads_bwd": (c_int, [_P, _P, _P, _P, _P, _P, _P, _P, c_int, c_int, c_int, c_int, _P]),
-  "iic_seg_head_workspace": (c_longlong, [c_int, c_int, c_int, c_int, c_int]),
+  "iic_cross_entropy": (c_int, [_P, _P, c_int, c_int, _P, _P, _P]),
+  "iic_linear_fwd": (c_int, [_P, _P, _P, _P, c_int, c_int, c_int, _P]),
+  "iic_linear_bwd": (c_int, [_P, _P, _P, _P, _P, _P, c_int, c_int, c_int, c_int, _P]),
+  "iic_col_sum": (c_int, [_P, c_int, c_longlong, c_int, _P, c_int, _P]),
+  "iic_seg_head_workspace":(c_longlong, [c_int, c_int, c_int, c_int, c_int]),
   "iic_seg_head_fwd": (c_int, [_P, c_int, _P, _P, _P, _P, c_int, c_int, c_int, c_int, c_int, c_int, c_int, _P]),
   "iic_seg_head_bwd": (c_int, [_P, c_int, _P, _P, _P, _P, _P, _P, _P, _P, c_int, c_int, c_int, c_int, c_int, c_int,
                                c_int, c_int, _P]),

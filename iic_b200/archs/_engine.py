@@ -591,6 +591,27 @@ class HeadsFunction(torch.autograd.Function):
     return dfeat, dw, db, None, None
 
 
+class LinearFunction(torch.autograd.Function):
+  """nn.Linear (fp32) without an activation: the `semisup` head of the TwoHead nets (net5g_two_head.py:22-24) and the last
+  Linear of SupHead5 (sup_head5.py:20) -- csrc/semisup.cu iic_linear_fwd / iic_linear_bwd."""
+
+  @staticmethod
+  def forward(ctx, x, w, b):
+    if not x.is_cuda:
+      raise RuntimeError("iic_b200 Linear heads run on CUDA tensors only (no CPU fallback)")
+    x = x.float().contiguous()
+    ctx.save_for_backward(x, w)
+    return K.linear_fwd(x, w.contiguous(), b.contiguous())
+
+  @staticmethod
+  def backward(ctx, dy):
+    x, w = ctx.saved_tensors
+    dw = torch.empty_like(w)
+    db = torch.empty(w.shape[0], device=w.device, dtype=torch.float32)
+    dx = K.linear_bwd(x, w.contiguous(), dy.contiguous().float(), dw, db, False, ctx.needs_input_grad[0])
+    return dx, dw, db
+
+
 class SubHeads(nn.Module):
   """num_sub_heads x (Linear(F -> k) + Softmax(dim=1)); parameters live at
   ``heads.{i}.0.{weight,bias}`` exactly like the reference's nn.Sequential(Linear, Softmax)."""

@@ -37,8 +37,12 @@ class ClusterNet5gTrunk(ResNetTrunk):
         for blk in layer:
           a = E.block_forward(ctx, blk, a)
       if penultimate_features:
-        assert not ctx.need_grad, "penultimate_features is an inference-only path"
-        return K.nhwc_to_nchw(a).reshape(a.shape[0], -1), None
+        # layer3 output flattened in NCHW order (net5g.py:58-60 of the reference); its fp32 gradient goes back to NHWC in
+        # the storage type, and the backward of the layer3 blocks runs unchanged (semisup finetuning, SupHead5)
+        n, h, w, c = a.shape
+        dt = ctx.dt
+        return (K.nhwc_to_nchw(a).reshape(n, -1),
+                (lambda dfeat: K.nchw_to_nhwc(dfeat.contiguous().float().reshape(n, c, h, w), dt)))
       for blk in self.layer4:
         a = E.block_forward(ctx, blk, a)
       n, h, w, c = a.shape

@@ -21,7 +21,7 @@ class ClusterNet5gTwoHeadHead(E.SubHeads):
   def forward(self, x, kmeans_use_features=False):
     if not self.semisup:
       return super().forward(x, kmeans_use_features=kmeans_use_features)
-    raise NotImplementedError("semisup (supervised cross-entropy) heads are outside the IIC hot path")
+    return E.LinearFunction.apply(x, self.head.weight, self.head.bias)  # logits, no softmax (the loss is cross-entropy)
 
 
 class ClusterNet5gTwoHead(ResNet):

@@ -20,7 +20,7 @@ class ClusterNet6cTwoHeadHead(E.SubHeads):
   def forward(self, x, kmeans_use_features=False):
     if not self.semisup:
       return super().forward(x, kmeans_use_features=kmeans_use_features)
-    raise NotImplementedError("semisup (supervised cross-entropy) heads are outside the IIC hot path")
+    return E.LinearFunction.apply(x, self.head.weight, self.head.bias)  # logits, no softmax (the loss is cross-entropy)
 
 
 class ClusterNet6cTwoHead(VGGNet):

@@ -126,51 +126,21 @@ __global__ void colsum_kernel(const float* __restrict__ a, float* __restrict__ o
 
 using namespace iic;
 
-// Split-K for the skinny head GEMMs (N = S*k = 50..350 columns, K = 512..4608): with one 64x64 tile per 64 rows the
-// ClusterNet6c logits (1400 x 4608 x 50) ran on 22 CTAs.  Partials in a per-device scratch, folded in split order.
-static float* heads_scratch(size_t bytes) {
+// Per-device split-K scratch of heads_gemm (simt_gemm.cuh): grown, never freed -- a captured CUDA graph
+// (iic_b200/graph.py) may hold the old pointer, and a later eager call with a larger batch (an evaluation pass between
+// graphed training steps) must not pull it from under the replays.
+float* iic::heads_scratch(size_t bytes) {
   static float* buf[64] = {nullptr};
   static size_t cap[64] = {0};
   int dev = 0;
   if (cudaGetDevice(&dev) != cudaSuccess || dev < 0 || dev >= 64) return nullptr;
   if (cap[dev] < bytes) {
-    // grown, never freed: a captured CUDA graph (iic_b200/graph.py) may hold the old pointer, and a later eager call with a
-    // larger batch (an evaluation pass between graphed training steps) must not pull it from under the replays
     float* nb = nullptr;
     if (cudaMalloc(&nb, bytes) != cudaSuccess) return nullptr;
     buf[dev] = nb;
     cap[dev] = bytes;
   }
   return buf[dev];
-}
-static int heads_splits(int M, int N, int K) {
-  const long long tiles = (long long)cdiv(M, ST_BM) * cdiv(N, ST_BN);
-  const int sms = device_sm_count();
-  if (tiles >= sms || K < 512) return 1;
-  long long s = (2ll * sms) / tiles;
-  if (s > K / 128) s = K / 128;
-  if (s > 32) s = 32;
-  return (int)(s < 1 ? 1 : s);
-}
-template <class AL, class BL, bool AK, bool BKC>
-static int heads_gemm(AL A, BL B, float* out, long long ldc, int M, int N, int K, cudaStream_t st) {
-  const int splits = heads_splits(M, N, K);
-  if (splits == 1 || ldc != N) {
-    StoreOut<float> St{out, nullptr, ldc};
-    return launch_simt<AL, BL, StoreOut<float>, AK, BKC>(A, B, St, M, N, K, 1, st);
-  }
-  float* ws = heads_scratch((size_t)splits * M * N * sizeof(float));
-  IIC_REQUIRE(ws != nullptr, IIC_ERR_CUDA, "heads: scratch allocation failed");
-  StorePartial Sp{ws};
-  int rc = launch_simt<AL, BL, StorePartial, AK, BKC>(A, B, Sp, M, N, K, splits, st);
-  if (rc != IIC_OK) return rc;
-  const long long count = (long long)M * N;
-  long long blocks = cdiv(count, 256);
-  if (blocks > 1024) blocks = 1024;
-  splitk_reduce_kernel<<<(int)blocks, 256, 0, st>>>(ws, out, count, splits, 0);
-  IIC_LAUNCH_CHECK();
-  count_launch();
-  return IIC_OK;
 }
 
 extern "C" int iic_heads_fwd(const float* feat, const float* w, const float* b, float* logits_ws, float* z, int n,

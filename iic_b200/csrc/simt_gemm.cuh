@@ -146,5 +146,40 @@ static inline int launch_simt(AL A, BL B, ST S, int M, int N, int K, int splits,
   return IIC_OK;
 }
 
+// ---- skinny dense GEMMs of the heads (conv_simt.cu: sub-heads; semisup.cu: Linear layers) ----------------------------
+// Split-K for the skinny head GEMMs (N = S*k = 10..350 columns, K = 512..4608): with one 64x64 tile per 64 rows the
+// ClusterNet6c logits (1400 x 4608 x 50) ran on 22 CTAs.  Partials in a per-device scratch (conv_simt.cu), folded in split
+// order.  accumulate != 0: out += A B^T instead of out = A B^T.
+float* heads_scratch(size_t bytes);
+
+static inline int heads_splits(int M, int N, int K) {
+  const long long tiles = (long long)cdiv(M, ST_BM) * cdiv(N, ST_BN);
+  const int sms = device_sm_count();
+  if (tiles >= sms || K < 512) return 1;
+  long long s = (2ll * sms) / tiles;
+  if (s > K / 128) s = K / 128;
+  if (s > 32) s = 32;
+  return (int)(s < 1 ? 1 : s);
+}
+template <class AL, class BL, bool AK, bool BKC>
+static int heads_gemm(AL A, BL B, float* out, long long ldc, int M, int N, int K, cudaStream_t st, int accumulate = 0) {
+  const int splits = heads_splits(M, N, K);
+  if (splits == 1 || ldc != N) {
+    StoreOut<float> St{out, accumulate ? out : nullptr, ldc};
+    return launch_simt<AL, BL, StoreOut<float>, AK, BKC>(A, B, St, M, N, K, 1, st);
+  }
+  float* ws = heads_scratch((size_t)splits * M * N * sizeof(float));
+  IIC_REQUIRE(ws != nullptr, IIC_ERR_CUDA, "heads: scratch allocation failed");
+  StorePartial Sp{ws};
+  int rc = launch_simt<AL, BL, StorePartial, AK, BKC>(A, B, Sp, M, N, K, splits, st);
+  if (rc != IIC_OK) return rc;
+  const long long count = (long long)M * N;
+  long long blocks = cdiv(count, 256);
+  if (blocks > 1024) blocks = 1024;
+  splitk_reduce_kernel<<<(int)blocks, 256, 0, st>>>(ws, out, count, splits, accumulate);
+  IIC_LAUNCH_CHECK();
+  count_launch();
+  return IIC_OK;
+}
 
 }  // namespace iic

@@ -745,6 +745,49 @@ def heads_bwd(feat, w, z, dz, S, k, want_dfeat):
   return dw, db, dfeat
 
 
+# ---- semi-supervised finetuning (csrc/semisup.cu) ------------------------------------------------
+@_cat("cross_entropy")
+def cross_entropy(logits, targets):
+  """logits [n, k] fp32, targets [n] int64 -> (mean NLL as a 0-dim fp32 tensor, dlogits [n, k] = (softmax - onehot) / n)."""
+  n, k = logits.shape
+  assert logits.dtype == torch.float32 and targets.dtype == torch.int64 and targets.shape == (n,)
+  loss = torch.empty((), device=logits.device, dtype=torch.float32)
+  dlogits = torch.empty_like(logits)
+  check(_lib.lib().iic_cross_entropy(_p(logits), _p(targets), n, k, _p(loss), _p(dlogits), _stream()), "iic_cross_entropy")
+  return loss, dlogits
+
+
+@_cat("linear")
+def linear_fwd(x, w, b):
+  """x [n, K], w [N, K], b [N] | None (fp32) -> y [n, N] = x w^T + b."""
+  n, K = x.shape
+  N = w.shape[0]
+  assert w.shape == (N, K) and x.dtype == w.dtype == torch.float32
+  y = torch.empty((n, N), device=x.device, dtype=torch.float32)
+  check(_lib.lib().iic_linear_fwd(_p(x), _p(w), _p(b), _p(y), n, K, N, _stream()), "iic_linear_fwd")
+  return y
+
+
+@_cat("linear")
+def linear_bwd(x, w, dy, dw, db, accumulate, want_dx):
+  """Writes (accumulate=False) or adds to dw [N, K] and db [N] | None; returns dx [n, K] or None."""
+  n, K = x.shape
+  N = w.shape[0]
+  assert dy.shape == (n, N) and dw.shape == (N, K)
+  dx = torch.empty_like(x) if want_dx else None
+  check(_lib.lib().iic_linear_bwd(_p(x), _p(w), _p(dy), _p(dw), _p(db), _p(dx), int(bool(accumulate)), n, K, N, _stream()),
+        "iic_linear_bwd")
+  return dx
+
+
+def col_sum(x, out, accumulate):
+  """out [C] (=|+=) column sums of x [..., C] (fp32 or bf16)."""
+  C = x.shape[-1]
+  check(_lib.lib().iic_col_sum(_p(x), iic_dtype(x), x.numel() // C, C, _p(out), int(bool(accumulate)), _stream()),
+        "iic_col_sum")
+  return out
+
+
 # ---- segmentation sub-head --------------------------------------------------------------------
 def seg_head_fwd(feat, w, H, W):
   """feat NHWC [n,hf,wf,C]; w [k,C] fp32 -> (out NCHW [n,k,H,W] fp32, zlow)"""

@@ -6,6 +6,8 @@ Clustering (code/scripts/cluster/cluster_sobel_twohead.py:286-355):
 Segmentation (code/scripts/segmentation/segmentation_twohead.py:262-361):
     zero_grad -> sobel_process(x, include_rgb), ... -> net(x, head), net(x_tf, head)
     -> IID_segmentation_loss(_uncollapsed) per sub-head with the batch's affine2_to_1 / mask, mean -> backward -> step
+Semi-supervised finetune (code/scripts/semisup/IID_semisup_STL10.py:241-256):
+    sobel_process(x) -> SupHead5 logits -> cross-entropy -> zero_grad (trunk, head) -> backward -> two Adam steps
 
 Inputs are the image batches the dataloaders hand to the script (host or device tensors; host tensors are copied on
 the current stream).  ``set_to_none=False`` is the reference's behaviour (torch 0.4.1 ``zero_grad`` zero-fills, so the
@@ -133,3 +135,30 @@ def iic_seg_step(net, optimiser, imgs, imgs_tf, affine2_to_1, mask_img1, head="B
   avg_loss.backward()
   _finish(net, optimiser, arena)
   return avg_loss.detach(), avg_loss_no_lamb.detach()
+
+
+def iic_semisup_step(net, optimisers, imgs, targets, penultimate_features=False, include_rgb=False, sobel=True, arena=None):
+  """One batch of the semi-supervised finetune (code/scripts/semisup/IID_semisup_STL10.py:241-256): sobel_process ->
+  net(imgs, penultimate_features) -> nn.CrossEntropyLoss() -> zero_grad of both optimisers -> backward -> opt_trunk.step(),
+  opt_head.step().  ``net`` is a SupHead5, ``optimisers`` the (opt_trunk, opt_head) pair of FusedAdam over
+  ``net.trunk.parameters()`` and ``net.head.parameters()``.  The sub-heads inside the trunk receive no gradient and are not
+  stepped, as in the reference.  Returns the loss as a 0-dim device tensor (no host sync)."""
+  from .utils.semisup.general import CrossEntropyLoss
+  opt_trunk, opt_head = optimisers
+  _zero(net, opt_trunk, arena, False, overlap=True)  # (every parameter gets its gradient from one backward node)
+  if arena is not None:
+    opt_head.grad_filter = arena.is_live
+  else:
+    opt_head.zero_grad(set_to_none=False)
+  dev = next(net.parameters()).device
+  if not imgs.is_cuda:
+    imgs = imgs.to(dev, non_blocking=True)
+  if not targets.is_cuda:
+    targets = targets.to(dev, non_blocking=True)
+  imgs = _to_net_input(imgs, sobel, include_rgb)
+  x_out = net(imgs, penultimate_features=penultimate_features)
+  loss = CrossEntropyLoss()(x_out, targets)
+  loss.backward()
+  _finish(net, opt_trunk, arena)
+  opt_head.step()
+  return loss.detach()

@@ -371,6 +371,26 @@ int iic_heads_fwd(const float* feat, const float* w, const float* b, float* logi
 int iic_heads_bwd(const float* feat, const float* w, const float* z, const float* dz, float* dlogits_ws,
                   float* dw, float* db, float* dfeat, int n, int F, int S, int k, void* stream);
 
+/* ---- a14: semi-supervised finetuning -- code/scripts/semisup/IID_semisup_STL10.py.
+ * iic_cross_entropy  nn.CrossEntropyLoss() with mean reduction (the criterion of IID_semisup_STL10.py:201, applied at
+ *                    :246) and its backward, in one launch.  logits [n][k] fp32, targets [n] int64 -> loss [1] fp32
+ *                    = mean_i (logsumexp(logits_i) - logits_i[t_i]) (stable log-sum-exp, fp64 sum folded in a fixed
+ *                    order: deterministic) and dlogits [n][k] = (softmax(logits) - onehot(t)) / n.  A target outside
+ *                    [0, k) makes the loss (and that row of dlogits) NaN; the call neither traps nor synchronises.
+ * iic_linear_fwd     nn.Linear: y [n][N] = x [n][K] w^T + b (w [N][K], b [N] or NULL), fp32 (the last Linear of
+ *                    SupHead5, sup_head5.py:20, and the `semisup` head of ClusterNet5gTwoHead / ClusterNet6cTwoHead,
+ *                    net5g_two_head.py:22-24, net6c_two_head.py:31-33).  No softmax.
+ * iic_linear_bwd     its backward: dw [N][K], db [N] (may be NULL) written (accumulate = 0) or added to (accumulate != 0);
+ *                    dx [n][K] overwritten when not NULL.
+ * iic_col_sum        out [cols] (=|+=) column sums of x [rows][cols] (`dtype` IIC_F32 / IIC_BF16): the bias gradient of
+ *                    SupHead5's first Linear (sup_head5.py:17), whose product runs as a 1x1 convolution. */
+int iic_cross_entropy(const float* logits, const long long* targets, int n, int k, float* loss, float* dlogits,
+                      void* stream);
+int iic_linear_fwd(const float* x, const float* w, const float* b, float* y, int n, int K, int N, void* stream);
+int iic_linear_bwd(const float* x, const float* w, const float* dy, float* dw, float* db, float* dx, int accumulate,
+                   int n, int K, int N, void* stream);
+int iic_col_sum(const void* x, int dtype, long long rows, int cols, float* out, int accumulate, void* stream);
+
 /* ---- a6: segmentation sub-heads -- code/archs/segmentation/net10a.py:34-59:
  *      Conv2d(C -> k, 1x1, padding=1, bias=False) -> Softmax2d -> F.interpolate(size=(H,W), bilinear,
  *      align_corners=False), one sub-head per call.
